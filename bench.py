@@ -20,6 +20,11 @@ evaluation at t0 + 2 ms, and one WeightedWbc QP.
 
 N>1 keeps the per-GPU instance count (weak scaling), sharded by contiguous blocks with no data-path collective; the per-instance
 torques are gathered to rank 0 with NCCL every step on a side stream.
+
+  --dump-outputs DIR   configs[1..3]: after the timed device-resident steps, rank 0 writes what the last step returned for its instances
+                       (xt, ut, info, sol, tau, status; info as columns alpha, merit0, merit1, viol0, viol1, armijo, status, n_trials)
+                       as DIR/<name>.npy in float64, rows in instance order, plus instance.npy (the global instance index of every row).
+                       Inputs depend only on the arguments, so two builds can be compared file by file.
 """
 import argparse
 import json
@@ -31,6 +36,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True      # the source tree may be read-only: nothing is written into it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -49,6 +55,22 @@ FP64_NOMINAL_TFLOPS = 37.0   # B200 FP64 CUDA-core peak (not in MEASURED_PEAKS.j
 GAIT_NAMES = ["stance", "trot", "standing_trot", "flying_trot"]
 GAIT_PERIOD = {"stance": 0.5, "trot": 0.6, "standing_trot": 0.6, "flying_trot": 0.4}
 KERNEL_OF = {"mpc_lq_project": "lq_kernel", "mpc_linearise": "lin_kernel", "mpc_riccati": "riccati_kernel", "mpc_forward_linesearch": "forward_linesearch2_kernel"}
+DUMP_LIMIT_BYTES = 64 * 2 ** 20
+
+
+def dump_outputs(path, outputs, instance):
+    """Write every [rows, ...] array of `outputs` and the row -> instance index as path/<name>.npy in float64. Above DUMP_LIMIT_BYTES in all,
+    every array keeps the same fixed, seeded sample of rows (configs[1] at its default size is written whole)."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in dict(outputs, instance=instance).items()}
+    rows = len(instance)
+    row_bytes = sum(a[:1].nbytes for a in arrays.values())
+    keep = min(rows, (DUMP_LIMIT_BYTES - 1024 * len(arrays)) // row_bytes)     # 1 KB per file covers the .npy header
+    if keep < rows:
+        sel = np.sort(np.random.default_rng(SEED).choice(rows, keep, replace=False))
+        arrays = {k: a[sel] for k, a in arrays.items()}
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 def load_peaks():
@@ -380,7 +402,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--torch-gather", action="store_true", help="multi-GPU: gather with torch.distributed instead of hb_shard_gather_dev")
     ap.add_argument("--e2e-chunks", type=int, default=0, help="chunks of the host-pointer cycle (0 = library default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy (configs[1..3])")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.config == 4):
+        ap.error("--dump-outputs applies to configs[1..3] of the b200 path")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
         run_reference(args, rank, world)
@@ -496,6 +523,13 @@ def main():
     launches = ctx.launch_count - l0
     prof = ctx.profile_read()
     ctx.profile_enable(False)
+    if args.dump_outputs and rank == 0:
+        info = d_info.cpu().numpy().view(hb.INFO_DTYPE)[:, 0]          # hb_solve_info records -> columns alpha ... armijo, status, n_trials
+        outs = {"xt": d_xt.cpu().numpy(), "ut": d_ut.cpu().numpy(), "info": np.stack([info[n] for n in hb.INFO_DTYPE.names], axis=1),
+                "sol": d_sol.cpu().numpy(), "tau": d_tau.cpu().numpy(), "status": d_st.cpu().numpy()}
+        if inv is not None:                 # back to instance order (configs[3])
+            outs = {k: v[inv] for k, v in outs.items()}
+        dump_outputs(args.dump_outputs, outs, np.arange(lo, hi))
     gather_ok = None
     if world > 1 and rank == 0:
         if shard is not None:

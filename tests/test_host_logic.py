@@ -4,6 +4,7 @@ with world_size 2 over gloo."""
 import ctypes as C
 import os
 import re
+import shutil
 import subprocess
 import sys
 
@@ -11,6 +12,7 @@ import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+HUNTER_CONFIG = os.path.join(ROOT, "tests", "golden", "hunter")        # hunter.urdf, task.info, reference.info of the original project
 
 
 def test_abi_exports_every_declared_symbol():
@@ -175,13 +177,9 @@ def test_task_info_parser_reads_the_wbc_estimator_and_solver_blocks():
 
 
 def test_task_info_parser_on_the_reference_file_when_present():
-    """The shipped task.info itself (only in the build container; the GPU box has no reference tree): the values equal the compiled-in defaults."""
-    import pytest
+    """The original project's shipped task.info (stored verbatim under tests/golden/hunter/): the values equal the compiled-in defaults."""
     import hunter_bipedal_control_b200 as hb
-    path = "/root/reference/legged_controllers/config/hunter/task.info"
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present")
-    ti = hb.parse_task_info(path)
+    ti = hb.parse_task_info(os.path.join(HUNTER_CONFIG, "task.info"))
     import ctypes as C
     d = hb.HbWbcSettings(); hb.load_library().hb_default_wbc_settings(C.byref(d))
     assert np.array_equal(ti.wbc.as_array(), d.as_array())
@@ -208,11 +206,13 @@ def test_native_shard_helpers_match_python_mirror():
 
 def test_model_constants_header_regenerates_from_the_reference_files_when_present(tmp_path):
     """include/hunter_model_constants.h (inertias, joint tree and limits from hunter.urdf; MPC / WBC weights and gains from task.info; default
-    joint state and gait templates from reference.info) is generated, not written by hand: regenerating it from the reference tree gives the
-    committed bytes (build container only; the GPU box has no reference tree)."""
-    ref = "/root/reference"
-    if not os.path.exists(os.path.join(ref, "legged_controllers/config/hunter/task.info")):
-        pytest.skip("reference tree not present")
+    joint state and gait templates from reference.info) is generated, not written by hand: regenerating it from the original project's files
+    (stored verbatim under tests/golden/hunter/, laid out here as in the original tree) gives the committed bytes."""
+    ref = tmp_path / "reference"
+    for name, rel in (("hunter.urdf", "legged_examples/legged_hunter/legged_hunter_description/urdf"), ("task.info", "legged_controllers/config/hunter"),
+                      ("reference.info", "legged_controllers/config/hunter")):
+        (ref / rel).mkdir(parents=True, exist_ok=True)
+        shutil.copyfile(os.path.join(HUNTER_CONFIG, name), ref / rel / name)
     out = tmp_path / "hunter_model_constants.h"
     r = subprocess.run([sys.executable, os.path.join(ROOT, "tools", "gen_model.py"), ref, str(out)], capture_output=True, text=True, timeout=120)
     assert r.returncode == 0, r.stderr[-2000:]
